@@ -64,6 +64,9 @@ def parse():
     ap.add_argument("--no-fps", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-vren-ops", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (per-ray rgb / opacity / depth / sample counts, the loss "
+                         "terms, the fp32 parameters after its Adam update) to DIR/<name>.npy, for comparing two builds")
     ap.add_argument("--ref-tcnn", default="fast", choices=["fast", "standin"],
                     help="--impl reference: which tinycudann stand-in drives the reference's Python (fast = performance-grade)")
     ap.add_argument("--ddp", default="auto", choices=["auto", "p2p", "nvls", "p2p_host", "nccl", "zero"],
@@ -372,24 +375,18 @@ def exchange_check(tr, world, rank):
 
 
 # --------------------------------------------------------------------------------------------------
-def run_b200(args):
-    import torch
-    from ngp_pl_b200 import _lib, synth
+def make_trainer(args, scene, world, rank, pg, dev):
+    """the workload's model, trainer and image bank in their seeded initial state"""
+    from ngp_pl_b200 import synth
     from ngp_pl_b200.models.networks import NGP
-    from ngp_pl_b200.models.rendering import render
-    from ngp_pl_b200.trainer import Trainer, shard_range
-    world, rank, local, pg = dist_setup()
-    dev = torch.device("cuda", local)
-    wl = WORKLOADS[args.workload]
-    n_rays = wl["n_rays"]
-    scene = make_scene(args.workload)
-    esf = scene.exp_step_factor
+    from ngp_pl_b200.trainer import Trainer
     bank = synth.RayBank(scene, n_images=N_TRAIN_IMAGES, device=dev, seed=rank)  # every rank: own images order/sampling
     # auto: the peer-load kernel up to 4 GPUs, the NVSwitch-reduced variant beyond (measured ms/step p2p vs nvls: N=2 0.390 vs
     # 0.425, N=4 0.381 vs 0.387, N=8 0.447 vs 0.431; profiles/r02_bench_n2_*.json, r02_exchange_residency.txt,
     # r02_bench_n8_*.json); falls back to p2p without a multicast mapping
     ddp_mode = args.ddp if args.ddp != "auto" else ("p2p" if world <= 4 else "nvls")
-    tkw = dict(n_rays=n_rays, lr=1e-2, exp_step_factor=esf, bg=(scene.bg,) * 3, process_group=pg, world_size=world, rank=rank, seed=rank)
+    tkw = dict(n_rays=WORKLOADS[args.workload]["n_rays"], lr=1e-2, exp_step_factor=scene.exp_step_factor, bg=(scene.bg,) * 3,
+               process_group=pg, world_size=world, rank=rank, seed=rank)
     model = NGP(scene.scale).to(dev)
     try:
         tr = Trainer(model, ddp=ddp_mode, **tkw)
@@ -402,6 +399,20 @@ def run_b200(args):
         tr = Trainer(model, ddp=fallback, **tkw)
         ddp_mode = ddp_note
     tr.attach_bank(bank)
+    return model, tr, bank, ddp_mode
+
+
+def run_b200(args):
+    import torch
+    from ngp_pl_b200 import _lib
+    from ngp_pl_b200.models.rendering import render
+    world, rank, local, pg = dist_setup()
+    dev = torch.device("cuda", local)
+    wl = WORKLOADS[args.workload]
+    n_rays = wl["n_rays"]
+    scene = make_scene(args.workload)
+    esf = scene.exp_step_factor
+    model, tr, bank, ddp_mode = make_trainer(args, scene, world, rank, pg, dev)
     xchk = exchange_check(tr, world, rank) if world > 1 else None
     pretrain = args.pretrain if args.pretrain is not None else 1000
     K, W = args.steps, max(args.warmup, 3)
@@ -457,14 +468,13 @@ def run_b200(args):
     for i in range(W):
         e2e_step(i)
     barrier(world)
-    Ke = min(K, 300)
     e0.record()
-    for i in range(Ke):
+    for i in range(K):
         e2e_step(i)
     e1.record()
     barrier(world)
     ms_e2e = max_over_ranks(e0.elapsed_time(e1), world)
-    e2e = {"value": world * n_rays * Ke / (ms_e2e * 1e-3), "unit": "rays/s", "steps": Ke,
+    e2e = {"value": world * n_rays * K / (ms_e2e * 1e-3), "unit": "rays/s", "steps": K,
            "h2d_bytes_per_step": n_rays * 9 * 4, "d2h_bytes_per_step": 32}
     tr.check_exchange()
 
@@ -568,6 +578,8 @@ def run_b200(args):
         except Exception as e:
             ops = {"unavailable": repr(e)}
 
+    if args.dump_outputs:
+        dump_outputs(args, scene, world, rank, pg, dev)
     if rank != 0:
         return
     line = {
@@ -604,6 +616,35 @@ def run_b200(args):
         except Exception as e:  # the oracle is only a reported baseline; never let it sink the bench line
             line["cpu_baseline"] = {"unavailable": repr(e)}
     print(json.dumps(line))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(args, scene, world, rank, pg, dev):
+    """What one step of the timed path (Trainer.capture + train_step) hands its caller, as float32 .npy files in
+    args.dump_outputs: per-ray rgb / opacity / depth / sample counts, the batch's target colours, the loss terms and the
+    fp32 parameters after the Adam update. The step runs on a fresh trainer in the workload's seeded initial state, so its
+    inputs are the same in every run and two builds can be compared output for output. (The trainer that was timed is not
+    used: its gradient scatter accumulates with float atomics, and over the pretraining steps Adam amplifies those
+    last-bit differences into a different trajectory in every run.) Rank 0 writes; every rank takes part in the step."""
+    import torch
+    _, tr, _, _ = make_trainer(args, scene, world, rank, pg, dev)
+    tr.capture(sample=True)
+    tr.train_step()
+    if world > 1:
+        tr.gather_master_params()
+    torch.cuda.synchronize()
+    if rank != 0:
+        return
+    out = {"rgb": tr.rgb, "opacity": tr.opacity, "depth": tr.depth, "n_samples": tr.n_samples, "loss_terms": tr.scalars,
+           "rgb_gt": tr.rgb_gt, "params": tr.P}
+    out = {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs of %d bytes exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES)
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(args.dump_outputs, k + ".npy"), a)
 
 
 def render_fps(render_fn, scene, dev, n_views, world=1, rank=0):

@@ -81,56 +81,34 @@ def test_encoder_network_forward_backward(oracle):
 
 @pytest.mark.parametrize("which", ["lego", "mip360"])
 def test_unmodified_reference_python_runs_on_our_vren_and_tcnn(which):
-    """the reference's own NGP / render / autograd Functions, bound to OUR vren and OUR tcnn"""
-    from oracle import ref_env
-    if not ref_env.python_available():
-        pytest.skip("reference python not staged (oracle/_ref/ngp_pl)")
+    """the reference's own NGP / render / autograd Functions, bound to OUR vren and OUR tcnn (stored in
+    tests/golden/parity_render.npz by tests/golden/make_golden_parity.py)"""
     from ngp_pl_b200 import synth
-    from ngp_pl_b200.models.networks import NGP
     from ngp_pl_b200.models.rendering import render
-    drop = ref_env.load_reference(drop_in=True)
-    scene = synth.lego_scene(0) if which == "lego" else synth.mip360_scene(0)
-    mine = NGP(scene.scale).cuda()
-    theirs = drop.NGP(scene.scale).cuda()  # reference class, our modules inside
-    g = torch.Generator().manual_seed(0)
-    with torch.no_grad():
-        p = mine.xyz_encoder.params
-        p[3072:] = ((torch.rand(p.numel() - 3072, generator=g) * 2 - 1) * 0.3).cuda()
-        mine.density_bitfield.copy_(torch.as_tensor(synth.pack_bits(synth.occupancy_grid(scene))).cuda())
-    theirs.load_state_dict({k: v.clone() for k, v in mine.state_dict().items()}, strict=True)
+    g = cases.golden("parity_render.npz")
+    pre = "dropin_%s_" % which
+    scene = cases.scene_by_name(which)
+    mine = cases.seeded_ngp(scene)
     o_np, d_np = cases.rays_from_scene(scene, 2048, 51, extra_edge_cases=False)
     o, d = torch.as_tensor(o_np).cuda(), torch.as_tensor(d_np).cuda()
     kw = {} if scene.exp_step_factor == 0 else {"exp_step_factor": scene.exp_step_factor}
     torch.manual_seed(5)
-    r_ref = drop.render(theirs, o, d, **kw)
-    torch.manual_seed(5)
     r_my = render(mine, o, d, **kw)
-    assert int(r_ref["rm_samples"]) == int(r_my["rm_samples"]) > 0
-    assert torch.equal(r_ref["rays_a"], r_my["rays_a"])
-    assert torch.equal(r_ref["ts"], r_my["ts"])
+    assert int(g[pre + "rm_samples"]) == int(r_my["rm_samples"]) > 0
+    assert cases.digest(r_my["rays_a"]) == str(g[pre + "rays_a"])
+    assert cases.digest(r_my["ts"]) == str(g[pre + "ts"])
     for k in ("rgb", "opacity", "depth"):
-        err = (r_ref[k].float() - r_my[k].float()).abs().max().item()
-        assert err < 3e-3 * max(1.0, r_ref[k].abs().max().item()), "%s differs by %g" % (k, err)
-    tgt = torch.rand(o.shape[0], 3, device="cuda")
-
-    def loss_of(res):
-        op = res["opacity"] + 1e-10
-        return ((res["rgb"] - tgt) ** 2).mean() + (1e-3 * (-op * torch.log(op))).mean()
-    theirs.zero_grad(); mine.zero_grad()
-    loss_of(r_ref).backward()
-    loss_of(r_my).backward()
-    for name in ("xyz_encoder.params", "rgb_net.params"):
-        ga = dict(theirs.named_parameters())[name].grad.float()
-        gb = dict(mine.named_parameters())[name].grad.float()
-        s = ga.abs().max().item()
-        assert s > 0 and (ga - gb).abs().max().item() < 0.05 * s, name
+        ref_k = g[pre + k]
+        err = np.abs(ref_k - r_my[k].detach().float().cpu().numpy()).max()
+        assert err < 3e-3 * max(1.0, np.abs(ref_k).max()), "%s differs by %g" % (k, err)
+    tgt = cases.render_target(o.shape[0])
+    op = r_my["opacity"] + 1e-10
+    mine.zero_grad()
+    (((r_my["rgb"] - tgt) ** 2).mean() + (1e-3 * (-op * torch.log(op))).mean()).backward()
+    cases.check_grads_vs_golden(mine, g, pre, 0.05)
     # test-time render through the reference's host loop on our operators vs our device-side wavefront
     K = synth.intrinsics(W=80, H=60, fx=1111.11 / 10)
     dirs = synth.ray_directions(K, "cuda")
     pose = torch.as_tensor(synth.camera_poses(3, radius=1.5 if which == "lego" else 0.9)[1]).cuda()
     o2, d2 = synth.get_rays(dirs, pose)
-    a = drop.render(theirs, o2, d2, test_time=True, **kw)
-    b = render(mine, o2, d2, test_time=True, **kw)
-    for k in ("rgb", "opacity", "depth"):
-        err = (a[k].float() - b[k].float()).abs()
-        assert err.max().item() < 2e-2 and err.mean().item() < 1e-3, k
+    cases.check_view_vs_golden(render(mine, o2, d2, test_time=True, **kw), g, pre + "view_")

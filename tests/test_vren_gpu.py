@@ -1,6 +1,7 @@
 """GPU parity of the twelve vren operators (through the C ABI) against
   (1) the CPU oracle (oracle/ngp_oracle.c) on the same seeded inputs, and
-  (2) the REAL reference kernels (oracle/_ref/vren) when they are present on the box.
+  (2) the REAL reference kernels on the same inputs, as stored in tests/golden/ (march_*.npz, composite.npz,
+      parity_ops.npz; arrays, or sha256 digests where the comparison is bit for bit).
 Marcher: per-ray sample counts and the t / dt / xyz sequences are BIT-EXACT.
 Compositing / distortion: 1e-4 relative (the reference uses __expf and serial fp32 sums).
 """
@@ -80,42 +81,35 @@ def test_aabb_and_march_train_vs_oracle(name, oracle):
 
 
 @pytest.mark.parametrize("name", cases.MARCH_CASES)
-def test_march_train_vs_reference_kernels(name, ref):
-    if ref is None:
-        pytest.skip("oracle/_ref not built on this box")
+def test_march_train_vs_reference_kernels(name):
     from ngp_pl_b200 import vren
+    g = cases.golden("march_%s.npz" % name)
     c = cases.march_case(name)
     o, d, bits, noise = T(c["o"]), T(c["d"]), T(c["bits"]), T(c["noise"])
     center = torch.zeros(1, 3, device="cuda")
     half = torch.full((1, 3), float(c["scale"]), device="cuda")
-    cnt_r, hits_r, _ = ref.vren.ray_aabb_intersect(o, d, center, half, 1)
     cnt_m, hits_m, _ = vren.ray_aabb_intersect(o, d, center, half, 1)
-    bits_equal(hits_m.cpu().numpy(), hits_r.cpu().numpy(), "ray_aabb_intersect hits_t")
-    assert (cnt_m == cnt_r).all()
+    bits_equal(hits_m.cpu().numpy(), g["hits_raw"], "ray_aabb_intersect hits_t")
+    assert (cnt_m.cpu().numpy() == g["hit_cnt"]).all()
     hits = near_clamp(hits_m)
     args = (o, d, hits, bits, c["cascades"], float(c["scale"]), float(c["esf"]), noise, 128, 1024)
-    ra_r, xyz_r, dir_r, dl_r, ts_r, cnt_r = ref.vren.raymarching_train(*args)
     ra_m, xyz_m, dir_m, dl_m, ts_m, cnt_m2 = vren.raymarching_train(*args)
-    assert int(cnt_r[0]) == int(cnt_m2[0])
-    ra_r = ra_r.cpu().numpy()
-    ra_r = ra_r[np.argsort(ra_r[:, 0], kind="stable")]
-    ra_m = ra_m.cpu().numpy()
-    assert (ra_r[:, 2] == ra_m[:, 2]).all(), "per-ray sample counts differ from the reference kernel"
-    sel = np.concatenate([np.arange(s, s + n) for _, s, n in ra_r if n > 0]) if int(cnt_r[0]) else np.zeros(0, np.int64)
     tot = int(cnt_m2[0])
-    bits_equal(ts_m[:tot].cpu().numpy(), ts_r.cpu().numpy()[sel], "ts vs reference")
-    bits_equal(dl_m[:tot].cpu().numpy(), dl_r.cpu().numpy()[sel], "deltas vs reference")
-    bits_equal(xyz_m[:tot].cpu().numpy(), xyz_r.cpu().numpy()[sel], "xyzs vs reference")
+    assert tot == int(g["total"])
+    assert (ra_m[:, 2].cpu().numpy() == g["counts"]).all(), "per-ray sample counts differ from the reference kernel"
+    bits_equal(ts_m[:tot].cpu().numpy(), g["ts"], "ts vs reference")
+    bits_equal(dl_m[:tot].cpu().numpy(), g["deltas"], "deltas vs reference")
+    bits_equal(xyz_m[:tot].cpu().numpy(), g["xyzs"], "xyzs vs reference")
 
 
 @pytest.mark.parametrize("name", cases.MARCH_CASES)
-def test_march_test_rounds(name, oracle, ref):
+def test_march_test_rounds(name, oracle):
     from ngp_pl_b200 import vren
+    g = cases.golden("parity_ops.npz")
     c = cases.march_case(name)
     o, d, bits = T(c["o"]), T(c["d"]), T(c["bits"])
     hits_np = cases.hits_for(c, oracle).copy()
     hits_m = T(hits_np)
-    hits_r = hits_m.clone()
     n = o.shape[0]
     alive = torch.arange(n, device="cuda")
     for ns in (1, 2, 4, 64):
@@ -126,49 +120,40 @@ def test_march_test_rounds(name, oracle, ref):
             bits_equal(a.cpu().numpy(), b, "raymarching_test %s (N_samples=%d)" % (nm, ns))
         assert (out_m[4].cpu().numpy() == out_o[4]).all()
         bits_equal(hits_m.cpu().numpy(), hits_np, "hits_t after round")
-        if ref is not None:
-            out_r = ref.vren.raymarching_test(o, d, hits_r, alive, bits, c["cascades"], float(c["scale"]), float(c["esf"]),
-                                              128, 1024, ns)
-            for a, b, nm in zip(out_m[:4], out_r[:4], ["xyzs", "dirs", "deltas", "ts"]):
-                bits_equal(a.cpu().numpy(), b.cpu().numpy(), "raymarching_test %s vs reference" % nm)
-            assert (out_m[4] == out_r[4]).all()
-            bits_equal(hits_m.cpu().numpy(), hits_r.cpu().numpy(), "hits_t vs reference")
+        key = "test_%s_%d_" % (name, ns)
+        for a, nm in zip(out_m[:4], ["xyzs", "dirs", "deltas", "ts"]):
+            assert cases.digest(a) == str(g[key + nm]), "raymarching_test %s (N_samples=%d) vs reference" % (nm, ns)
+        assert cases.digest(out_m[4].long()) == str(g[key + "neff"]), "N_eff_samples vs reference"
+        assert cases.digest(hits_m) == str(g[key + "hits"]), "hits_t vs reference"
 
 
-def test_march_large_vs_reference(ref):
+def test_march_large_vs_reference():
     """bit-exactness over many rays (size-independent check at the bench's ray count and beyond)"""
-    if ref is None:
-        pytest.skip("oracle/_ref not built on this box")
     from ngp_pl_b200 import synth, vren
-    for scene, esf, n_rays in ((synth.lego_scene(0), 0.0, 1 << 18), (synth.mip360_scene(0), 1.0 / 256, 1 << 16)):
+    g = cases.golden("parity_ops.npz")
+    for which, esf, n_rays in cases.LARGE_MARCH:
+        pre = "large_%s_" % which
+        scene = cases.scene_by_name(which)
         bits = T(synth.pack_bits(synth.occupancy_grid(scene)))
         o_np, d_np = cases.rays_from_scene(scene, n_rays, 77)
         o, d = T(o_np), T(d_np)
         center = torch.zeros(1, 3, device="cuda")
         half = torch.full((1, 3), scene.scale, device="cuda")
         _, hits_m, _ = vren.ray_aabb_intersect(o, d, center, half, 1)
-        _, hits_r, _ = ref.vren.ray_aabb_intersect(o, d, center, half, 1)
-        assert torch.equal(hits_m.view(torch.int32), hits_r.view(torch.int32))
+        assert cases.digest(hits_m) == str(g[pre + "hits"]), "%s: ray_aabb_intersect vs reference" % which
         hits = near_clamp(hits_m)
         noise = torch.rand(n_rays, device="cuda", generator=torch.Generator("cuda").manual_seed(5))
         args = (o, d, hits, bits, scene.cascades, scene.scale, esf, noise, 128, 1024)
-        ra_r, xyz_r, _, dl_r, ts_r, cnt_r = ref.vren.raymarching_train(*args)
         ra_m, xyz_m, _, dl_m, ts_m, cnt_m = vren.raymarching_train(*args)
         tot = int(cnt_m[0])
-        assert tot == int(cnt_r[0]) and tot > 0
-        order = torch.argsort(ra_r[:, 0])
-        ra_r = ra_r[order]
-        assert torch.equal(ra_r[:, 2], ra_m[:, 2])
-        # gather the reference's samples into ray order
-        seg = torch.repeat_interleave(torch.arange(n_rays, device="cuda"), ra_m[:, 2])
-        within = torch.arange(tot, device="cuda") - ra_m[:, 1][seg]
-        src = ra_r[:, 1][seg] + within
-        assert torch.equal(ts_m[:tot].view(torch.int32), ts_r[src].view(torch.int32))
-        assert torch.equal(dl_m[:tot].view(torch.int32), dl_r[src].view(torch.int32))
-        assert torch.equal(xyz_m[:tot].view(torch.int32), xyz_r[src].view(torch.int32))
+        assert tot == int(g[pre + "total"]) and tot > 0
+        assert cases.digest(ra_m[:, 2].long()) == str(g[pre + "counts"]), "%s: per-ray sample counts vs reference" % which
+        # the reference's samples are stored gathered into ray order
+        for t, nm in ((ts_m, "ts"), (dl_m, "deltas"), (xyz_m, "xyzs")):
+            assert cases.digest(t[:tot]) == str(g[pre + nm]), "%s: %s vs reference" % (which, nm)
 
 
-def test_composite_train_fw_bw(oracle, ref):
+def test_composite_train_fw_bw(oracle):
     from ngp_pl_b200 import vren
     c = cases.composite_case()
     sig, rgbs, dl, ts, ra = T(c["sigmas"]), T(c["rgbs"]), T(c["deltas"]), T(c["ts"]), T(c["rays_a"])
@@ -187,32 +172,22 @@ def test_composite_train_fw_bw(oracle, ref):
     rel_close(drgbs.cpu().numpy(), o_drgbs, atol=1e-5, what="dL_drgbs")
     # dL_dsigmas is a difference of O(1) terms scaled by delta: absolute floor = 1e-4 * delta * |terms|
     rel_close(dsig.cpu().numpy(), o_dsig, atol=1e-5, what="dL_dsigmas")
-    if ref is not None:
-        r_total, r_op, r_dp, r_rgb, r_ws = ref.vren.composite_train_fw(sig, rgbs, dl, ts, ra, thr)
-        assert torch.equal(r_total, total)
-        rel_close(opacity.cpu().numpy(), r_op.cpu().numpy(), what="opacity vs reference")
-        rel_close(rgb.cpu().numpy(), r_rgb.cpu().numpy(), what="rgb vs reference")
-        rel_close(depth.cpu().numpy(), r_dp.cpu().numpy(), what="depth vs reference")
-        rel_close(ws.cpu().numpy(), r_ws.cpu().numpy(), atol=2e-6, what="ws vs reference")
-        r_dsig, r_drgbs = ref.vren.composite_train_bw(T(c["dO"]), T(c["dD"]), T(c["dC"]), T(c["dws"]), sig, rgbs, r_ws, dl, ts,
-                                                      ra, r_op, r_dp, r_rgb, thr)
-        rel_close(drgbs.cpu().numpy(), r_drgbs.cpu().numpy(), atol=1e-5, what="dL_drgbs vs reference")
-        rel_close(dsig.cpu().numpy(), r_dsig.cpu().numpy(), atol=1e-5, what="dL_dsigmas vs reference")
+    g = cases.golden("composite.npz")
+    assert (total.cpu().numpy() == g["total"]).all()
+    rel_close(opacity.cpu().numpy(), g["opacity"], what="opacity vs reference")
+    rel_close(rgb.cpu().numpy(), g["rgb"], what="rgb vs reference")
+    rel_close(depth.cpu().numpy(), g["depth"], what="depth vs reference")
+    rel_close(ws.cpu().numpy(), g["ws"], atol=2e-6, what="ws vs reference")
+    rel_close(drgbs.cpu().numpy(), g["drgbs"], atol=1e-5, what="dL_drgbs vs reference")
+    rel_close(dsig.cpu().numpy(), g["dsig"], atol=1e-5, what="dL_dsigmas vs reference")
 
 
-def test_composite_test_fw(oracle, ref):
+def test_composite_test_fw(oracle):
     from ngp_pl_b200 import vren
-    rng = np.random.RandomState(4)
-    n_rays, n_alive, ns = 200, 150, 8
-    alive_np = rng.permutation(n_rays)[:n_alive].astype(np.int64)
-    sig = np.exp(rng.normal(0, 2.5, (n_alive, ns))).astype(np.float32)
-    rgbs = rng.rand(n_alive, ns, 3).astype(np.float32)
-    dl = np.full((n_alive, ns), 0.01, np.float32)
-    ts = np.cumsum(dl, 1).astype(np.float32)
-    neff = rng.randint(0, ns + 1, n_alive).astype(np.int32)
-    op0 = (rng.rand(n_rays) * 0.9).astype(np.float32)
-    dp0 = rng.rand(n_rays).astype(np.float32)
-    rgb0 = rng.rand(n_rays, 3).astype(np.float32)
+    c = cases.composite_test_case()
+    alive_np, sig, rgbs, dl, ts, neff = c["alive"], c["sigmas"], c["rgbs"], c["deltas"], c["ts"], c["neff"]
+    op0, dp0, rgb0 = c["opacity"], c["depth"], c["rgb"]
+    n_rays = op0.shape[0]
     alive_m, op_m, dp_m, rgb_m = T(alive_np), T(op0), T(dp0), T(rgb0)
     hits = torch.zeros(n_rays, 2, device="cuda")
     vren.composite_test_fw(T(sig), T(rgbs), T(dl), T(ts), hits, alive_m, 1e-2, T(neff), op_m, dp_m, rgb_m)
@@ -222,15 +197,13 @@ def test_composite_test_fw(oracle, ref):
     rel_close(op_m.cpu().numpy(), op_o, what="opacity")
     rel_close(dp_m.cpu().numpy(), dp_o, what="depth")
     rel_close(rgb_m.cpu().numpy(), rgb_o, what="rgb")
-    if ref is not None:
-        alive_r, op_r, dp_r, rgb_r = T(alive_np), T(op0), T(dp0), T(rgb0)
-        ref.vren.composite_test_fw(T(sig), T(rgbs), T(dl), T(ts), hits, alive_r, 1e-2, T(neff), op_r, dp_r, rgb_r)
-        assert torch.equal(alive_r, alive_m)
-        rel_close(op_m.cpu().numpy(), op_r.cpu().numpy(), what="opacity vs reference")
-        rel_close(rgb_m.cpu().numpy(), rgb_r.cpu().numpy(), what="rgb vs reference")
+    g = cases.golden("parity_ops.npz")
+    assert (alive_m.cpu().numpy() == g["ctest_alive"]).all()
+    rel_close(op_m.cpu().numpy(), g["ctest_opacity"], what="opacity vs reference")
+    rel_close(rgb_m.cpu().numpy(), g["ctest_rgb"], what="rgb vs reference")
 
 
-def test_distortion_loss(oracle, ref):
+def test_distortion_loss(oracle):
     from ngp_pl_b200 import vren
     c = cases.composite_case(seed=9)
     _, _, _, _, ws_np = oracle.composite_train_fw(c["sigmas"], c["rgbs"], c["deltas"], c["ts"], c["rays_a"], 1e-4)
@@ -245,15 +218,14 @@ def test_distortion_loss(oracle, ref):
     dws = vren.distortion_loss_bw(T(dL), wi, wti, ws, dl, ts, ra)
     o_dws = oracle.distortion_bw(dL, o_wi, o_wti, ws_np, c["deltas"], c["ts"], c["rays_a"])
     rel_close(dws.cpu().numpy(), o_dws, atol=3e-5, what="dL_dws")
-    if ref is not None:
-        r_loss, r_wi, r_wti = ref.vren.distortion_loss_fw(ws, dl, ts, ra)
-        rel_close(loss.cpu().numpy(), r_loss.cpu().numpy(), atol=3e-5, what="distortion loss vs reference")
-        r_dws = ref.vren.distortion_loss_bw(T(dL), r_wi, r_wti, ws, dl, ts, ra)
-        rel_close(dws.cpu().numpy(), r_dws.cpu().numpy(), atol=3e-5, what="dL_dws vs reference")
+    g = cases.golden("parity_ops.npz")
+    rel_close(loss.cpu().numpy(), g["dist_loss"], atol=3e-5, what="distortion loss vs reference")
+    rel_close(dws.cpu().numpy(), g["dist_dws"], atol=3e-5, what="dL_dws vs reference")
 
 
-def test_packbits_morton(oracle, ref):
+def test_packbits_morton(oracle):
     from ngp_pl_b200 import vren
+    gold = cases.golden("parity_ops.npz")
     rng = np.random.RandomState(21)
     for dtype in (torch.float32, torch.float16, torch.float64):
         grid = rng.normal(0, 1, 4096 * 8).astype(np.float32)
@@ -262,10 +234,7 @@ def test_packbits_morton(oracle, ref):
         vren.packbits(g, 0.25, bf)
         want = oracle.packbits(g.float().cpu().numpy(), 0.25) if dtype != torch.float64 else oracle.packbits(grid, 0.25)
         assert (bf.cpu().numpy() == want).all()
-        if ref is not None:
-            bf2 = torch.zeros_like(bf)
-            ref.vren.packbits(g, 0.25, bf2)
-            assert torch.equal(bf, bf2)
+        assert cases.digest(bf) == str(gold["packbits_" + str(dtype).split(".")[1]]), "packbits %s vs reference" % dtype
     # odd size (not a multiple of 4 bytes) takes the byte path
     grid = rng.normal(0, 1, 1001 * 8).astype(np.float32)
     bf = torch.zeros(1001, dtype=torch.uint8, device="cuda")
@@ -278,10 +247,10 @@ def test_packbits_morton(oracle, ref):
     assert (m.cpu().numpy() == oracle.morton3D(coords)).all()
     inv = vren.morton3D_invert(m)
     assert (inv.cpu().numpy() == coords).all()
-    if ref is not None:
-        c128 = T(rng.randint(0, 128, (5000, 3)).astype(np.int32))
-        assert torch.equal(vren.morton3D(c128), ref.vren.morton3D(c128))
-        assert torch.equal(vren.morton3D_invert(vren.morton3D(c128)), ref.vren.morton3D_invert(ref.vren.morton3D(c128)))
+    c128 = T(rng.randint(0, 128, (5000, 3)).astype(np.int32))
+    m = vren.morton3D(c128)
+    assert cases.digest(m.long()) == str(gold["morton128"]), "morton3D vs reference"
+    assert cases.digest(vren.morton3D_invert(m).long()) == str(gold["morton128_invert"]), "morton3D_invert vs reference"
 
 
 def test_empty_and_error_paths():
